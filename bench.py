@@ -7,6 +7,7 @@ Metric (BASELINE.json): prove ms for a 2^20-step trace at default 120-bit ProofO
   python bench.py [--gpus N] [--steps K] [--warmup W]             our arm (CUDA prover)
   python bench.py --impl reference [--steps K] [--warmup W]       reference arm: the CPU restatement of the reference
                                                                   prover (oracle/, single thread) on a bounded sample
+  --dump-outputs DIR (our arm): also write the proof of the last timed step to DIR/<name>.npy (see dump_outputs)
 Workload: the reference's collatz example (src/examples/collatz.rs) with a start value whose trajectory has 2600 steps,
 which the VM turns into 548k operations => a trace of 2^20 steps x 26 registers.
 N > 1: one process per GPU (torchrun); ONE proof is sharded over the N ranks by LDE coset ranges (DESIGN.md section 7): every
@@ -144,6 +145,17 @@ def log_n_of(n):
     return int(n).bit_length() - 1
 
 
+def dump_outputs(out_dir, proof):
+    """--dump-outputs: what a caller of prove_device receives from the last timed proof, one DIR/<name>.npy per field, so that two
+    builds can be compared output for output.  Every field is a byte string (the nonce as its 8 little-endian bytes), stored as one
+    float32 element per byte, which is exact."""
+    os.makedirs(out_dir, exist_ok=True)
+    fields = {"proof": proof.bytes, "trace_root": proof.trace_root, "constraint_root": proof.constraint_root, "pow_seed": proof.pow_seed,
+              "pow_nonce": proof.pow_nonce.to_bytes(8, "little")}
+    for name, data in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.frombuffer(data, dtype=np.uint8).astype(np.float32))
+
+
 def golden_for(log_n):
     try:
         g = json.load(open(os.path.join(ROOT, "tests", "golden", "collatz_2_%d.json" % log_n)))
@@ -268,6 +280,8 @@ def run_ours(args):
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
     total_dev_ms = float(np.sum(dev_ms))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, proof)
 
     # end-to-end: host trace (pinned) -> proof bytes on the host, through the public API call a user makes
     e2e_ms = []
@@ -559,7 +573,12 @@ def main():
     ap.add_argument("--microbench", action="store_true", help="BASELINE config 5: NTT / LDE / leaf hash / Merkle sweep instead of the proof benchmark")
     ap.add_argument("--quick", action="store_true", help="--microbench: three sizes only")
     ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step to DIR/<name>.npy (float32, one element per byte)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.microbench or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the CUDA prover benchmark only")
     if args.microbench:
         out = run_microbench(args)
         if out is not None:
