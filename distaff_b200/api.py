@@ -7,10 +7,20 @@ import numpy as np
 from . import backend, felt, hostvm
 
 
-class ProofOptions:
-    """stark::ProofOptions (options.rs:29-50): same argument checks, same defaults (options.rs:82-91)."""
+# hashes a proof can commit with (dg_options_t.hash_id); the others cannot hash a trace row (include/distaff_gpu.h)
+PROOF_HASHES = {"blake3": 0, "sha3": 4}
 
-    def __init__(self, extension_factor=32, num_queries=50, grinding_factor=20):
+
+class ProofOptions:
+    """stark::ProofOptions (options.rs:29-50): same argument checks, same defaults (options.rs:82-91).  hash_fn is "blake3" (the
+    default) or "sha3" (SHA3-256, hash.rs:212-218)."""
+
+    def __init__(self, extension_factor=32, num_queries=50, grinding_factor=20, hash_fn="blake3"):
+        if hash_fn not in PROOF_HASHES:
+            if hash_fn in ("rescue", "poseidon", "gmimc"):
+                raise ValueError(f"hash_fn {hash_fn!r} cannot commit to a proof: it absorbs at most 64 bytes and a trace row is longer "
+                                 "(the reference panics in build_merkle_tree); use 'blake3' or 'sha3'")
+            raise ValueError(f"unknown hash_fn {hash_fn!r}: use 'blake3' or 'sha3'")
         assert extension_factor & (extension_factor - 1) == 0, "extension_factor must be a power of 2"
         assert extension_factor >= 16, "extension_factor cannot be smaller than 16"
         assert extension_factor <= 256, "extension_factor cannot be greater than 256"
@@ -20,9 +30,10 @@ class ProofOptions:
         self.extension_factor = extension_factor
         self.num_queries = num_queries
         self.grinding_factor = grinding_factor
+        self.hash_fn = hash_fn
 
     def _c(self):
-        return backend.DgOptions(self.extension_factor, self.num_queries, self.grinding_factor, 0)
+        return backend.DgOptions(self.extension_factor, self.num_queries, self.grinding_factor, PROOF_HASHES[self.hash_fn])
 
 
 class StarkProof:
@@ -92,7 +103,8 @@ def prove_device(d_registers, width, length, ctx_depth, loop_depth, public_input
 
 def verify(program_hash, public_inputs, outputs, proof):
     """distaff::verify (lib.rs:68-75 -> stark/verifier.rs:11-75) on the GPU.  Returns None when the proof is accepted, otherwise the
-    reference's error string (what `Err(msg)` carries); raises DgError for bytes that are not a serialized StarkProof."""
+    reference's error string (what `Err(msg)` carries); raises DgError for bytes that are not a serialized StarkProof.  The hash
+    (blake3 or sha3) is the one the proof's options name: the last byte of the bytes."""
     data = proof.bytes if isinstance(proof, StarkProof) else bytes(proof)
     fi, fo = felt.from_ints(public_inputs), felt.from_ints(outputs)
     msg = ctypes.create_string_buffer(256)
@@ -137,11 +149,11 @@ def lde(values, blowup=32):
     return out
 
 
-HASH_IDS = {"blake3": 0, "rescue": 1, "poseidon": 2}
+HASH_IDS = {"blake3": 0, "rescue": 1, "poseidon": 2, "sha3": 4}
 
 
 def merkle_build(leaves, hash="blake3"):
-    """crypto::build_merkle_nodes (merkle.rs:269-294): bytes (n*32) -> bytes (n*32), heap layout; hash in blake3 | rescue | poseidon"""
+    """crypto::build_merkle_nodes (merkle.rs:269-294): bytes (n*32) -> bytes (n*32), heap layout; hash in blake3 | rescue | poseidon | sha3"""
     leaves = bytes(leaves)
     n = len(leaves) // 32
     out = ctypes.create_string_buffer(n * 32)
@@ -153,7 +165,7 @@ def merkle_build(leaves, hash="blake3"):
 
 
 def hash64(messages, hash="rescue"):
-    """crypto::hash::{blake3, rescue, poseidon} of n independent 64-byte messages: bytes (n*64) -> bytes (n*32)"""
+    """crypto::hash::{blake3, rescue, poseidon, sha3} of n independent 64-byte messages: bytes (n*64) -> bytes (n*32)"""
     messages = bytes(messages)
     assert len(messages) % 64 == 0
     n = len(messages) // 64

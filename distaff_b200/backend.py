@@ -81,6 +81,7 @@ EXPORTS = {
     "dg_host_prng_vector": [vp, u64, vp],
     "dg_host_query_positions": [vp, u64, u32, u32, vp],
     "dg_host_blake3": [vp, ctypes.c_size_t, vp],
+    "dg_host_sha3": [vp, ctypes.c_size_t, vp],
     "dg_host_plan_batch": [vp, u32, u64, vp, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)],
     "dg_host_merkle_verify_plan": [vp, u32, u32, u32, vp, u32, vp, ctypes.c_size_t, vp, vp, ctypes.c_size_t, vp, vp],
     "dg_host_periodic_tables": [vp],

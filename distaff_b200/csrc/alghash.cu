@@ -1,4 +1,5 @@
-// Algebraic hash functions over F_M on the GPU: Rescue and Poseidon, one thread per 64-byte message, and Merkle trees built with them.
+// Algebraic hash functions over F_M on the GPU: Rescue and Poseidon, one thread per 64-byte message, and Merkle trees built with them
+// (and with BLAKE3 or SHA3-256, the hashes a proof commits with, under the same interface).
 //
 // Replaces (SURVEY.md section 8 row a10, micro-benchmark config C5)
 //   hash::rescue     /root/reference/src/crypto/hash.rs:151-177
@@ -16,7 +17,7 @@
 #define DG_MUL_CALL 1
 #include "common.cuh"
 #include "air_constants.h"
-#include "blake3.cuh"
+#include "digest.cuh"
 
 namespace dg {
 
@@ -96,11 +97,12 @@ template <int HASH>
 __global__ void __launch_bounds__(128) alg_hash64_kernel(const uint4 *__restrict__ in, uint4 *__restrict__ out, unsigned long long n) {
     const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    if (HASH == 0) {
+    if (HASH == DG_HASH_BLAKE3 || HASH == DG_HASH_SHA3) {
         uint32_t m[16], cv[8];
 #pragma unroll
         for (int q = 0; q < 4; q++) { const uint4 v = in[4 * i + q]; m[4 * q] = v.x; m[4 * q + 1] = v.y; m[4 * q + 2] = v.z; m[4 * q + 3] = v.w; }
-        b3::hash64(m, cv);
+        if (HASH == DG_HASH_SHA3) Sha3Hash::hash64(m, cv);
+        else Blake3Hash::hash64(m, cv);
         out[2 * i] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
         out[2 * i + 1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
         return;
@@ -119,13 +121,14 @@ __global__ void __launch_bounds__(128) alg_hash64_kernel(const uint4 *__restrict
 }
 
 void alg_hash64(Context &c, int hash_id, const void *in, void *out, unsigned long long n) {
-    DG_REQUIRE(hash_id >= 0 && hash_id <= 2, "hash id must be 0 (blake3), 1 (rescue) or 2 (poseidon)");
+    DG_REQUIRE((hash_id >= 0 && hash_id <= 2) || hash_id == DG_HASH_SHA3, "hash id must be 0 (blake3), 1 (rescue), 2 (poseidon) or 4 (sha3)");
     if (n == 0) return;
     alg_upload_constants(c);
     const unsigned grid = (unsigned)((n + 127) / 128);
     switch (hash_id) {
         case 0: alg_hash64_kernel<0><<<grid, 128, 0, c.stream>>>((const uint4 *)in, (uint4 *)out, n); break;
         case 1: alg_hash64_kernel<1><<<grid, 128, 0, c.stream>>>((const uint4 *)in, (uint4 *)out, n); break;
+        case DG_HASH_SHA3: alg_hash64_kernel<DG_HASH_SHA3><<<grid, 128, 0, c.stream>>>((const uint4 *)in, (uint4 *)out, n); break;
         default: alg_hash64_kernel<2><<<grid, 128, 0, c.stream>>>((const uint4 *)in, (uint4 *)out, n); break;
     }
     c.launches++;

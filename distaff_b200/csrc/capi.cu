@@ -5,15 +5,8 @@
 #include "host_fs.h"
 #include "shard.h"
 #include "poly.h"
+#include "digest.cuh"
 #include <thread>
-
-namespace dg {
-void hash_trace_rows(Context &c, const fe *ext, void *leaves, int w, int log_n, int log_blowup);
-void merkle_build(Context &c, const void *leaves, void *nodes, unsigned long long L);
-unsigned long long pow_search(Context &c, const uint8_t seed[32], unsigned grinding);
-void pow_hash(const uint8_t seed[32], unsigned long long nonce, uint8_t out[32]);
-void hash_rows_plain(Context &c, const fe *cols, void *digests, int w, unsigned long long rows);
-}  // namespace dg
 
 namespace dg {
 std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::vector<fe> &inputs, const std::vector<fe> &outputs,
@@ -217,7 +210,7 @@ int dg_dev_merkle_build(const void *d_leaves, uint64_t n_leaves, void *d_nodes, 
         Context &c = ctx();
         std::lock_guard<std::mutex> lk(c.mu);
         EventTimer t(c.stream, ms);
-        merkle_build(c, d_leaves, d_nodes, n_leaves);
+        merkle_build<Blake3Hash>(c, d_leaves, d_nodes, n_leaves);
         t.stop();
         DG_CUDA(cudaStreamSynchronize(c.stream));
     });
@@ -238,7 +231,7 @@ int dg_dev_hash_rows(const void *d_ext, uint32_t width, uint32_t log_n, uint32_t
         std::lock_guard<std::mutex> lk(c.mu);
         DG_REQUIRE(width >= 1 && width < 128, "width must be in 1..127");
         EventTimer t(c.stream, ms);
-        hash_trace_rows(c, (const fe *)d_ext, d_leaves, (int)width, (int)log_n, (int)log_blowup);
+        hash_trace_rows<Blake3Hash>(c, (const fe *)d_ext, d_leaves, (int)width, (int)log_n, (int)log_blowup);
         t.stop();
         DG_CUDA(cudaStreamSynchronize(c.stream));
     });
@@ -284,7 +277,7 @@ int dg_merkle_build(const uint8_t *leaves, uint64_t n_leaves, uint8_t *nodes) {
         DG_REQUIRE(n_leaves >= 2 && (n_leaves & (n_leaves - 1)) == 0, "number of leaves must be a power of 2 and >= 2");
         DevBuf d_l(n_leaves * 32), d_n(n_leaves * 32);
         DG_CUDA(cudaMemcpyAsync(d_l.p, leaves, n_leaves * 32, cudaMemcpyHostToDevice, c.stream));
-        merkle_build(c, d_l.p, d_n.p, n_leaves);
+        merkle_build<Blake3Hash>(c, d_l.p, d_n.p, n_leaves);
         DG_CUDA(cudaMemcpyAsync(nodes, d_n.p, n_leaves * 32, cudaMemcpyDeviceToHost, c.stream));
         DG_CUDA(cudaStreamSynchronize(c.stream));
     });
@@ -293,7 +286,7 @@ int dg_hash64(int hash, const uint8_t *messages64, uint64_t n, uint8_t *digests3
     return guarded([&] {
         Context &c = ctx();
         std::lock_guard<std::mutex> lk(c.mu);
-        DG_REQUIRE(hash >= 0 && hash <= 2, "hash id must be 0 (blake3), 1 (rescue) or 2 (poseidon)");
+        DG_REQUIRE((hash >= 0 && hash <= 2) || hash == DG_HASH_SHA3, "hash id must be 0 (blake3), 1 (rescue), 2 (poseidon) or 4 (sha3)");
         if (n == 0) return;
         DG_REQUIRE(messages64 && digests32, "null buffer");
         DevBuf d_in(n * 64), d_out(n * 32);
@@ -324,7 +317,7 @@ int dg_hash_rows(const uint8_t *columns, uint32_t width, uint64_t rows, uint8_t 
         DevBuf d_c((size_t)width * rows * 16), d_d(rows * 32);
         DG_CUDA(cudaMemcpyAsync(d_c.p, columns, (size_t)width * rows * 16, cudaMemcpyHostToDevice, c.stream));
         // reuse the trace-row kernel with a single "coset": physical position == logical row
-        hash_rows_plain(c, d_c.as<fe>(), d_d.p, (int)width, rows);
+        hash_rows_plain<Blake3Hash>(c, d_c.as<fe>(), d_d.p, (int)width, rows);
         DG_CUDA(cudaMemcpyAsync(digests, d_d.p, rows * 32, cudaMemcpyDeviceToHost, c.stream));
         DG_CUDA(cudaStreamSynchronize(c.stream));
     });
@@ -335,9 +328,9 @@ int dg_find_pow_nonce(const uint8_t seed[32], uint32_t grinding_factor, uint64_t
         std::lock_guard<std::mutex> lk(c.mu);
         DG_REQUIRE(seed && nonce, "null argument");
         DG_REQUIRE(grinding_factor <= 32, "grinding factor cannot be greater than 32");
-        unsigned long long n = pow_search(c, seed, grinding_factor);
+        unsigned long long n = pow_search<Blake3Hash>(c, seed, grinding_factor);
         *nonce = n;
-        if (new_seed) pow_hash(seed, n, new_seed);
+        if (new_seed) pow_hash<Blake3Hash>(seed, n, new_seed);
     });
 }
 int dg_field_op(int op, int impl, const uint8_t *a, const uint8_t *b, uint8_t *out, uint64_t n) {
@@ -465,6 +458,9 @@ int dg_host_query_positions(const uint8_t seed[32], uint64_t domain_size, uint32
     });
 }
 int dg_host_blake3(const uint8_t *data, size_t len, uint8_t out32[32]) { return guarded([&] { fs::blake3_short(data, len, out32); }); }
+int dg_host_sha3(const uint8_t *data, size_t len, uint8_t out32[32]) {
+    return guarded([&] { DG_REQUIRE(out32 && (data || len == 0), "null argument"); fs::sha3_256(data, len, out32); });
+}
 int dg_host_plan_batch(const uint64_t *indexes, uint32_t n_indexes, uint64_t n_leaves, uint64_t *out, size_t cap, size_t *written) {
     return guarded([&] {
         DG_REQUIRE(indexes && out && written, "null argument");

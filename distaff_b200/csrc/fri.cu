@@ -12,10 +12,11 @@
 // and 1/x is a power of the inverse LDE root (table lookup): no field inversion is needed.  The interpolating cubic is
 // unique and the arithmetic exact, hence the values equal the reference's.
 #include "poly.h"
-#include "blake3.cuh"
+#include "digest.cuh"
 
 namespace dg {
 
+template <class H>
 __global__ void __launch_bounds__(256) fri_hash_rows_kernel(const fe *__restrict__ v, Layout in, Layout rows, uint4 *__restrict__ leaves) {
     const unsigned long long R = 1ULL << rows.log_d;
     const unsigned long long t = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -27,15 +28,18 @@ __global__ void __launch_bounds__(256) fri_hash_rows_kernel(const fe *__restrict
         const uint4 x = reinterpret_cast<const uint4 *>(v)[in.phys(r + (unsigned long long)j * R)];
         m[4 * j] = x.x; m[4 * j + 1] = x.y; m[4 * j + 2] = x.z; m[4 * j + 3] = x.w;
     }
-    b3::hash64(m, cv);
+    H::hash64(m, cv);
     leaves[2 * r] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
     leaves[2 * r + 1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
 }
+template <class H>
 void fri_hash_rows(Context &c, const fe *values, Layout in, Layout rows, void *leaves) {
     const unsigned long long R = 1ULL << rows.log_d;
-    fri_hash_rows_kernel<<<(unsigned)((R + 255) / 256), 256, 0, c.stream>>>(values, in, rows, (uint4 *)leaves); c.launches++;
+    fri_hash_rows_kernel<H><<<(unsigned)((R + 255) / 256), 256, 0, c.stream>>>(values, in, rows, (uint4 *)leaves); c.launches++;
     DG_CUDA(cudaGetLastError());
 }
+template void fri_hash_rows<Blake3Hash>(Context &, const fe *, Layout, Layout, void *);
+template void fri_hash_rows<Sha3Hash>(Context &, const fe *, Layout, Layout, void *);
 
 // special_x = field::prng(layer root) (fri/prover.rs:29) derived on the device, so that a layer's fold does not wait for a round trip
 // to the host: StdRng::from_seed(root) = ChaCha20 (64-bit block counter, stream 0), Uniform(0..M) = widening multiply of a 128-bit
@@ -112,6 +116,7 @@ void fri_fold(Context &c, const fe *values, Layout in, fe *next, Layout out, con
 // ---- coset-sharded layers (multi-GPU): a rank holds the cosets [c0, c0 + 2^log_nc) of a layer of 2^log_d values as the slab
 //      [c - c0][k], k < 2^(log_d - log_b).  Row r = b k' + c and its three companions r + jR (R = D/4) have k = k' + j R/b inside the
 //      same coset, so hashing and folding need no other rank's data; the folded value of row r is element k' of coset c of the next layer.
+template <class H>
 __global__ void __launch_bounds__(256) fri_hash_rows_local_kernel(const fe *__restrict__ v, int log_d, int log_b, int log_nc, uint4 *__restrict__ items) {
     const int log_kr = log_d - 2 - log_b;                       // rows per coset
     const unsigned long long total = 1ULL << (log_kr + log_nc);
@@ -125,16 +130,19 @@ __global__ void __launch_bounds__(256) fri_hash_rows_local_kernel(const fe *__re
         const uint4 x = col[(unsigned long long)j << log_kr];
         m[4 * j] = x.x; m[4 * j + 1] = x.y; m[4 * j + 2] = x.z; m[4 * j + 3] = x.w;
     }
-    b3::hash64(m, cv);
+    H::hash64(m, cv);
     const unsigned long long it = (kp << log_nc) + cl;        // ShardedTree item layout [k'][c - c0]
     items[2 * it] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
     items[2 * it + 1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
 }
+template <class H>
 void fri_hash_rows_local(Context &c, const fe *values_local, int log_d, int log_b, int log_nc, void *items_local) {
     const unsigned long long total = 1ULL << (log_d - 2 - log_b + log_nc);
-    fri_hash_rows_local_kernel<<<(unsigned)((total + 255) / 256), 256, 0, c.stream>>>(values_local, log_d, log_b, log_nc, (uint4 *)items_local); c.launches++;
+    fri_hash_rows_local_kernel<H><<<(unsigned)((total + 255) / 256), 256, 0, c.stream>>>(values_local, log_d, log_b, log_nc, (uint4 *)items_local); c.launches++;
     DG_CUDA(cudaGetLastError());
 }
+template void fri_hash_rows_local<Blake3Hash>(Context &, const fe *, int, int, int, void *);
+template void fri_hash_rows_local<Sha3Hash>(Context &, const fe *, int, int, int, void *);
 
 __global__ void __launch_bounds__(256) fri_fold_local_kernel(const fe *__restrict__ v, int log_d, int log_b, int log_nc, unsigned c0, fe *__restrict__ next,
                                                              const fe *__restrict__ alpha_p, TwiddleRef inv_root, int shift, fe tau_inv, fe inv4) {

@@ -6,6 +6,7 @@
 #include <stdexcept>
 #include "air_constants.h"
 #include "blake3.cuh"
+#include "keccak.cuh"
 
 namespace dg {
 namespace fs {
@@ -97,6 +98,24 @@ void blake3_short(const uint8_t *data, size_t len, uint8_t out[32]) {
         b3::compress(cv, m, 0, (uint32_t)take, flags);
     }
     memcpy(out, cv, 32);
+}
+
+// ---- SHA3-256 ---------------------------------------------------------------------------------------------------------------
+void sha3_256(const uint8_t *data, size_t len, uint8_t out[32]) {
+    uint64_t a[25] = {0};
+    for (size_t off = 0;; off += 136) {                          // 136-byte blocks; the last one (possibly empty) carries the padding
+        uint8_t block[136] = {0};
+        const size_t take = off < len ? std::min<size_t>(136, len - off) : 0;
+        if (take) memcpy(block, data + off, take);
+        const bool last = take < 136;
+        if (last) { block[take] ^= 0x06; block[135] ^= 0x80; }
+        for (int i = 0; i < 17; i++) { uint64_t v; memcpy(&v, block + 8 * i, 8); a[i] ^= v; }
+        sha3::keccak_f(a);
+        if (last) break;
+    }
+    uint32_t o[8];
+    sha3::squeeze(a, o);
+    memcpy(out, o, 32);
 }
 
 // ---- coefficients ----------------------------------------------------------------------------------------------------------

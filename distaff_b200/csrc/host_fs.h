@@ -46,6 +46,8 @@ bool rng_hooks_active();
 
 // ---- BLAKE3 of a short message (<= 1024 bytes) on the host -------------------------------------------------------------
 void blake3_short(const uint8_t *data, size_t len, uint8_t out[32]);
+// ---- SHA3-256 of a message of any length on the host (keccak.cuh) ---------------------------------------------------------
+void sha3_256(const uint8_t *data, size_t len, uint8_t out[32]);
 
 // ---- constraint coefficients, arranged for the evaluation kernel --------------------------------------------------------
 struct ConstraintCoefficients {

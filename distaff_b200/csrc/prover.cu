@@ -4,6 +4,7 @@
 // the PCIe bus after the register traces have been uploaded.
 #include "prover.h"
 #include "air.h"
+#include "digest.cuh"
 #include "host_fs.h"
 #include "poly.h"
 #include "shard.h"
@@ -204,13 +205,13 @@ private:
 };
 
 // d_regs: register traces in device memory; when `host_cols` is given they are not there yet: column chunks are uploaded on the
-// copy stream while the previous chunk is being interpolated and extended (the upload hides behind the LDE)
-static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols, uint32_t width, uint64_t length, uint32_t ctx_depth,
-                         uint32_t loop_depth, const uint8_t *inputs16, uint32_t n_inputs, const uint8_t *outputs16, uint32_t n_outputs,
-                         const dg_options_t &opt, dg_prove_stats_t *stats) {
+// copy stream while the previous chunk is being interpolated and extended (the upload hides behind the LDE); H: the commitment hash
+template <class H>
+static Proof *prove_pipeline(Context &c, fe *d_regs, const uint8_t *const *host_cols, uint32_t width, uint64_t length, uint32_t ctx_depth,
+                             uint32_t loop_depth, const uint8_t *inputs16, uint32_t n_inputs, const uint8_t *outputs16, uint32_t n_outputs,
+                             const dg_options_t &opt, dg_prove_stats_t *stats) {
     // ---- argument checks (trace_table.rs:23-58, options.rs:29-50, lib.rs:33-34) -----------------------------------------------
     const uint64_t n = length, b = opt.extension_factor;
-    DG_REQUIRE(opt.hash_id == 0, "unsupported hash function (only blake3 is serialisable, options.rs:107)");
     DG_REQUIRE(b >= 16 && b <= 256 && (b & (b - 1)) == 0, "extension_factor must be a power of 2 between 16 and 256");
     DG_REQUIRE(opt.num_queries > 0 && opt.num_queries <= 128, "num_queries must be in 1..128");
     DG_REQUIRE(opt.grinding_factor <= 32, "grinding factor cannot be greater than 32");
@@ -320,10 +321,10 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
     clk.mark(1);
     sub.mark("1.lde");
     DevBuf t_leaves(N_loc * 32);
-    hash_trace_rows(c, ext.as<fe>(), t_leaves.p, w, log_n, log_nc);          // local rows, [k][c - c0]
+    hash_trace_rows<H>(c, ext.as<fe>(), t_leaves.p, w, log_n, log_nc);          // local rows, [k][c - c0]
     sub.mark("2.hash_rows");
     ShardedTree t_tree;
-    t_tree.build(c, t_leaves.p, n, log_nc);
+    t_tree.build<H>(c, t_leaves.p, n, log_nc);
     memcpy(proof->trace_root, t_tree.root.data(), 32);
 
     // ---- 3: evaluate constraints --------------------------------------------------------------------------------------------------------
@@ -425,10 +426,10 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
     DevBuf c_ext(N_loc * 16), c_items((N_loc / 4) * 32);
     lde_batch(c, combined.as<fe>(), c_ext.as<fe>(), log_n, log_b, 8, 1, E, N_loc, c0, (unsigned)nc);
     sub.mark("5.lde");
-    constraint_items_local(c, c_ext.as<fe>(), log_n, log_nc, c_items.p);      // first tree level: H(4 evaluations), [k][c4 local]
+    constraint_items_local<H>(c, c_ext.as<fe>(), log_n, log_nc, c_items.p);      // first tree level: H(4 evaluations), [k][c4 local]
     sub.mark("5.items");
     ShardedTree c_tree;
-    c_tree.build(c, c_items.p, n, log_nc - 2);
+    c_tree.build<H>(c, c_items.p, n, log_nc - 2);
     memcpy(proof->constraint_root, c_tree.root.data(), 32);
 
     // ---- 6: DEEP composition polynomial ---------------------------------------------------------------------------------------------------------
@@ -530,8 +531,8 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
             if (local) {
                 // rows r = b k' + c of the own cosets: hashes in ShardedTree order, n' = R / b subtrees of nc leaves per rank
                 L.leaves.alloc((R >> log_g) * 32);
-                fri_hash_rows_local(c, cur, lay.log_d, log_b, log_nc, L.leaves.p);
-                L.tree.build(c, L.leaves.p, R >> log_b, log_nc, false);
+                fri_hash_rows_local<H>(c, cur, lay.log_d, log_b, log_nc, L.leaves.p);
+                L.tree.build<H>(c, L.leaves.p, R >> log_b, log_nc, false);
                 const fe *alpha = folding_point(L.tree.root_dev(), li);
                 L.folded.alloc((R >> log_g) * 16);
                 fri_fold_local(c, cur, lay.log_d, log_b, log_nc, c0, L.folded.as<fe>(), alpha, inv_root, log_N, tau_inv, inv4);
@@ -541,8 +542,8 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
             }
             const Layout rows{log_r, (lay.log_b >= 0 && log_r >= lay.log_b) ? lay.log_b : -1};
             L.leaves.alloc(R * 32); L.nodes.alloc(R * 32);
-            fri_hash_rows(c, cur, lay, rows, L.leaves.p);
-            merkle_build(c, L.leaves.p, L.nodes.p, R);
+            fri_hash_rows<H>(c, cur, lay, rows, L.leaves.p);
+            merkle_build<H>(c, L.leaves.p, L.nodes.p, R);
             if (R * 4 <= 256) {                                    // MAX_REMAINDER_LENGTH (fri/mod.rs:13): the remainder's root only
                 DG_REQUIRE(li < (size_t)MAX_LAYERS, "too many FRI layers");
                 DG_CUDA(cudaMemcpyAsync((uint8_t *)d_roots.p + 32 * li, (const uint8_t *)L.nodes.p + 32, 32, cudaMemcpyDeviceToDevice, c.stream));
@@ -568,9 +569,9 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
         for (auto &L : layers) roots.insert(roots.end(), L.root.begin(), L.root.end());
         uint8_t seed[32];
         debug_dump_host("fri_roots", roots.data(), roots.size());
-        fs::blake3_short(roots.data(), roots.size(), seed);
-        proof->pow_nonce = pow_search(c, seed, opt.grinding_factor);
-        pow_hash(seed, proof->pow_nonce, proof->pow_seed);
+        H::message(roots.data(), roots.size(), seed);
+        proof->pow_nonce = pow_search<H>(c, seed, opt.grinding_factor);
+        pow_hash<H>(seed, proof->pow_nonce, proof->pow_seed);
         try {
             positions = fs::query_positions(proof->pow_seed, N, b, opt.num_queries);
         } catch (const std::exception &e) { throw Error(DG_ERR_EXHAUSTED, e.what()); }
@@ -705,7 +706,7 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
         out.u64(rem_off.size());
         for (size_t off : rem_off) out.felt(fb.value(off));
         out.u64(proof->pow_nonce);
-        out.u8((uint8_t)log_b); out.u8((uint8_t)opt.num_queries); out.u8((uint8_t)opt.grinding_factor); out.u8(0);
+        out.u8((uint8_t)log_b); out.u8((uint8_t)opt.num_queries); out.u8((uint8_t)opt.grinding_factor); out.u8((uint8_t)H::id);
     }
     clk.mark(9);
     sub.mark("9.openings");
@@ -719,6 +720,16 @@ static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols
         stats->kernel_launches = c.launches - launches0;
     }
     return guard.release();
+}
+
+static Proof *prove_core(Context &c, fe *d_regs, const uint8_t *const *host_cols, uint32_t width, uint64_t length, uint32_t ctx_depth,
+                         uint32_t loop_depth, const uint8_t *inputs16, uint32_t n_inputs, const uint8_t *outputs16, uint32_t n_outputs,
+                         const dg_options_t &opt, dg_prove_stats_t *stats) {
+    if (const char *why = proof_hash_error(opt.hash_id)) throw Error(DG_ERR_INVALID, why);
+    return with_proof_hash(opt.hash_id, [&](auto h) {
+        return prove_pipeline<decltype(h)>(c, d_regs, host_cols, width, length, ctx_depth, loop_depth, inputs16, n_inputs, outputs16, n_outputs,
+                                           opt, stats);
+    });
 }
 
 Proof *prove_device(Context &c, const fe *d_regs, uint32_t width, uint64_t length, uint32_t ctx_depth, uint32_t loop_depth,

@@ -1,5 +1,5 @@
 #include "shard.h"
-#include "blake3.cuh"
+#include "digest.cuh"
 #include "poly.h"
 
 namespace dg {
@@ -37,9 +37,9 @@ ShardLocation ShardGeom::node(uint64_t h) const {
 
 // ---- kernels ------------------------------------------------------------------------------------------------------------------
 // levels of a heap-layout tree from L/2 nodes down to (and including) the level with `stop` nodes (hash.cu)
-void merkle_levels_down_to(Context &c, const void *leaves, void *nodes, unsigned long long L, unsigned long long stop);
+template <class H>
 void merkle_build_partial(Context &c, const void *leaves, void *nodes, unsigned long long L, unsigned long long stop) {
-    merkle_levels_down_to(c, leaves, nodes, L, stop);
+    merkle_levels_down_to<H>(c, leaves, nodes, L, stop);
 }
 
 // upper[(n << log_g) + (k << log_g) + g] = gathered[g][k]
@@ -58,6 +58,7 @@ void interleave_roots(Context &c, const void *gathered, void *upper, unsigned lo
 }
 
 // items[k * (nc/4) + c4] = H(ev[4c4][k], ev[4c4+1][k], ev[4c4+2][k], ev[4c4+3][k]) over the local cosets (prover.rs:84-86,180-187)
+template <class H>
 __global__ void __launch_bounds__(256) constraint_items_kernel(const fe *__restrict__ ev, int log_n, int log_nc, uint4 *__restrict__ items) {
     const unsigned long long n = 1ULL << log_n;
     const unsigned long long total = n << (log_nc - 2);
@@ -71,17 +72,19 @@ __global__ void __launch_bounds__(256) constraint_items_kernel(const fe *__restr
         const uint4 x = reinterpret_cast<const uint4 *>(ev)[(4 * c4 + u) * n + k];
         m[4 * u] = x.x; m[4 * u + 1] = x.y; m[4 * u + 2] = x.z; m[4 * u + 3] = x.w;
     }
-    b3::hash64(m, cv);
+    H::hash64(m, cv);
     items[2 * j] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
     items[2 * j + 1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
 }
+template <class H>
 void constraint_items_local(Context &c, const fe *evals_local, int log_n, int log_nc, void *items) {
     const unsigned long long total = (1ULL << log_n) << (log_nc - 2);
-    constraint_items_kernel<<<(unsigned)((total + 255) / 256), 256, 0, c.stream>>>(evals_local, log_n, log_nc, (uint4 *)items); c.launches++;
+    constraint_items_kernel<H><<<(unsigned)((total + 255) / 256), 256, 0, c.stream>>>(evals_local, log_n, log_nc, (uint4 *)items); c.launches++;
     DG_CUDA(cudaGetLastError());
 }
 
 // ---- sharded tree -------------------------------------------------------------------------------------------------------------------
+template <class H>
 void ShardedTree::build(Context &c, const void *items_local_dev, uint64_t n, int log_blk, bool fetch_root) {
     int log_g = 0;
     while ((1 << log_g) < c.world) log_g++;
@@ -92,14 +95,14 @@ void ShardedTree::build(Context &c, const void *items_local_dev, uint64_t n, int
         // one rank: the local heap is the whole tree; the mid and top heaps alias it (their indices are global heap indices then)
         DG_REQUIRE(local_items >= 2, "tree needs at least 2 items");
         local_nodes.alloc(local_items * 32);
-        merkle_build(c, items_local_dev, local_nodes.p, local_items);
+        merkle_build<H>(c, items_local_dev, local_nodes.p, local_items);
         mid_p = top_p = local_nodes.p;
     } else {
         DG_REQUIRE(n >= G && n % G == 0, "sharded tree needs at least one block per rank and k-range");
         const void *roots = items_local_dev;
         if (log_blk > 0) {
             local_nodes.alloc(local_items * 32);
-            merkle_build_partial(c, items_local_dev, local_nodes.p, local_items, n);
+            merkle_build_partial<H>(c, items_local_dev, local_nodes.p, local_items, n);
             roots = (const uint8_t *)local_nodes.p + n * 32;           // heap level with n nodes: the subtree roots, by k
         }
         // re-shard the roots by k-range: recv[g'][k'] = root (k = g n/G + k') of rank g'
@@ -110,10 +113,10 @@ void ShardedTree::build(Context &c, const void *items_local_dev, uint64_t n, int
         if (c.mark) c.mark("tree.a2a");
         mid.alloc(2 * n * 32);
         interleave_roots(c, recv.p, mid.p, chunk, log_g);           // mid[n + k' G + g'] : nodes [g n, (g + 1) n) of the global level n G
-        merkle_finish(c, mid.p, n);                                 // mid[1] = global node G + g
+        merkle_finish<H>(c, mid.p, n);                                 // mid[1] = global node G + g
         top.alloc(2 * G * 32);
         comm_all_gather(c, (const uint8_t *)mid.p + 32, (uint8_t *)top.p + G * 32, 32);
-        merkle_finish(c, top.p, G);
+        merkle_finish<H>(c, top.p, G);
         if (c.mark) c.mark("tree.mid+top");
         mid_p = mid.p; top_p = top.p;
     }
@@ -122,6 +125,10 @@ void ShardedTree::build(Context &c, const void *items_local_dev, uint64_t n, int
         DG_CUDA(cudaStreamSynchronize(c.stream));
     }
 }
+template void ShardedTree::build<Blake3Hash>(Context &, const void *, uint64_t, int, bool);
+template void ShardedTree::build<Sha3Hash>(Context &, const void *, uint64_t, int, bool);
+template void constraint_items_local<Blake3Hash>(Context &, const fe *, int, int, void *);
+template void constraint_items_local<Sha3Hash>(Context &, const fe *, int, int, void *);
 
 // out[t] = base_t ? ((const uint4 *)base_t)[unit_t] : 0
 __global__ void fetch_units_kernel(const unsigned long long *__restrict__ req, unsigned count, uint4 *__restrict__ out) {

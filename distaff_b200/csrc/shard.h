@@ -71,8 +71,8 @@ struct ShardedTree {
     const void *mid_p = nullptr, *top_p = nullptr;     // one rank: both alias the local heap (global heap indices)
     Digest root;
 
-    // fetch_root = false leaves the root on the device (upper_p + 32): no host synchronisation
-    void build(Context &c, const void *items_local_dev, uint64_t n, int log_blk, bool fetch_root = true);
+    // fetch_root = false leaves the root on the device (upper_p + 32): no host synchronisation; H = the proof's hash (digest.cuh)
+    template <class H> void build(Context &c, const void *items_local_dev, uint64_t n, int log_blk, bool fetch_root = true);
     const void *root_dev() const { return (const uint8_t *)top_p + 32; }
     // locations as references for a FetchBatch
     FetchRef item_ref(uint64_t item_index) const { ShardLocation l = geom.item(item_index); return FetchRef{items_local, l.index, l.owner}; }
@@ -84,10 +84,10 @@ struct ShardedTree {
     }
 };
 
-void merkle_build_partial(Context &c, const void *leaves, void *nodes, unsigned long long L, unsigned long long stop);
-void merkle_build(Context &c, const void *leaves, void *nodes, unsigned long long L);
-void merkle_finish(Context &c, void *nodes, unsigned long long m);
+template <class H> void merkle_build_partial(Context &c, const void *leaves, void *nodes, unsigned long long L, unsigned long long stop);
+template <class H> void merkle_build(Context &c, const void *leaves, void *nodes, unsigned long long L);
+template <class H> void merkle_finish(Context &c, void *nodes, unsigned long long m);
 void interleave_roots(Context &c, const void *gathered, void *upper, unsigned long long n, int log_g);
-void constraint_items_local(Context &c, const fe *evals_local, int log_n, int log_nc, void *items);   // [k][c4_local] digests
+template <class H> void constraint_items_local(Context &c, const fe *evals_local, int log_n, int log_nc, void *items);   // [k][c4_local] digests
 
 }  // namespace dg

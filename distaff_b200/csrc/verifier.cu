@@ -9,7 +9,7 @@
 // query positions, coefficients, FRI folding points) and turns every batch-Merkle verification into a plan of (left, right, out)
 // hashing steps per tree level -- pure index logic, following verify_batch statement by statement, including its use of the current
 // level's position as the slot of `proof.nodes` -- while the device does all of the arithmetic and hashing in five launches:
-//   1. BLAKE3 of the opened trace rows and of the opened FRI rows (the Merkle leaves),
+//   1. the hash (BLAKE3 or SHA3-256, from the proof's options) of the opened trace rows and of the opened FRI rows (the Merkle leaves),
 //   2. all Merkle plans at once (one block per tree, one barrier per level),
 //   3. the transition constraints at the out-of-domain point z: the prover's own constraint kernel (air.cu) in verify mode, with the
 //      deep values as its two rows, the cycle polynomials evaluated at z^(n/16) and the powers z^inc from the host,
@@ -22,17 +22,13 @@
 #include <map>
 #include <set>
 #include "air.h"
-#include "blake3.cuh"
+#include "digest.cuh"
 #include "host_fs.h"
 #include "poly.h"
 #include "prover.h"
 #include "shard.h"
 
 namespace dg {
-
-void hash_rows_plain(Context &c, const fe *cols, void *digests, int w, unsigned long long rows);
-void hash64_contiguous(Context &c, const void *in, void *out, unsigned long long count);
-void pow_hash(const uint8_t seed[32], unsigned long long nonce, uint8_t out[32]);
 
 namespace {
 
@@ -200,6 +196,7 @@ MerklePlan plan_verify_batch(const std::vector<uint64_t> &indexes_in, int depth,
 struct TreeDesc { uint32_t ops_base, n_levels, levels_base, pad; };
 
 // one block per tree: ops of a level in parallel, levels separated by barriers
+template <class H>
 __global__ void __launch_bounds__(128) merkle_verify_kernel(uint4 *pool, const uint32_t *__restrict__ ops, const uint32_t *__restrict__ level_start,
                                                             const TreeDesc *__restrict__ trees) {
     const TreeDesc t = trees[blockIdx.x];
@@ -211,7 +208,7 @@ __global__ void __launch_bounds__(128) merkle_verify_kernel(uint4 *pool, const u
             const uint4 l0 = pool[2 * (size_t)op[0]], l1 = pool[2 * (size_t)op[0] + 1], r0 = pool[2 * (size_t)op[1]], r1 = pool[2 * (size_t)op[1] + 1];
             m[0] = l0.x; m[1] = l0.y; m[2] = l0.z; m[3] = l0.w; m[4] = l1.x; m[5] = l1.y; m[6] = l1.z; m[7] = l1.w;
             m[8] = r0.x; m[9] = r0.y; m[10] = r0.z; m[11] = r0.w; m[12] = r1.x; m[13] = r1.y; m[14] = r1.z; m[15] = r1.w;
-            b3::hash64(m, cv);
+            H::hash64(m, cv);
             pool[2 * (size_t)op[2]] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
             pool[2 * (size_t)op[2] + 1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
         }
@@ -320,12 +317,10 @@ bool host_plan_verify_batch(const std::vector<uint64_t> &indexes, int depth, siz
     return true;
 }
 
-// returns "" when the proof is accepted, the reference's error string otherwise; throws Error for malformed input / CUDA failures
-std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::vector<fe> &inputs, const std::vector<fe> &outputs,
-                         const uint8_t *proof_bytes, size_t proof_len) {
-    ParsedProof P;
-    if (!parse_proof(proof_bytes, proof_len, P)) throw Error(DG_ERR_INVALID, "malformed proof bytes (bincode layout of StarkProof, proof.rs:10-37)");
-    if (P.hash_id != 0) return "unsupported hash function";
+namespace {
+template <class H>
+std::string verify_parsed(Context &c, const ParsedProof &P, const uint8_t program_hash[32], const std::vector<fe> &inputs,
+                          const std::vector<fe> &outputs) {
     DG_REQUIRE(P.log_ext >= 4 && P.log_ext <= 8, "invalid extension factor in proof options");
     DG_REQUIRE(P.domain_depth >= P.log_ext + 4 && P.domain_depth <= 30, "invalid domain depth");
     DG_REQUIRE(inputs.size() <= 8 && outputs.size() <= 8, "cannot have more than 8 public inputs / outputs");
@@ -340,8 +335,8 @@ std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::
     fri_roots.insert(fri_roots.end(), P.rem_root.begin(), P.rem_root.end());
     DG_REQUIRE(fri_roots.size() <= 1024, "too many FRI layers");
     uint8_t seed[32], pseed[32];
-    fs::blake3_short(fri_roots.data(), fri_roots.size(), seed);
-    pow_hash(seed, P.pow_nonce, pseed);
+    H::message(fri_roots.data(), fri_roots.size(), seed);
+    pow_hash<H>(seed, P.pow_nonce, pseed);
     {
         uint64_t o0;
         memcpy(&o0, pseed, 8);
@@ -403,7 +398,7 @@ std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::
     std::vector<fe> rows_cm((size_t)w * nq);                       // column-major [w][nq]
     for (int q = 0; q < nq; q++) for (int j = 0; j < w; j++) rows_cm[(size_t)j * nq + q] = P.trace_evaluations[q][j];
     const fe *rows_dev = upload(c, d_rows, rows_cm);
-    hash_rows_plain(c, rows_dev, pool_dev + 2 * (size_t)tv_base, w, nq);
+    hash_rows_plain<H>(c, rows_dev, pool_dev + 2 * (size_t)tv_base, w, nq);
     std::vector<fe> fri_rows;
     std::vector<unsigned long long> fri_pos;
     std::vector<unsigned> fri_layer;
@@ -419,7 +414,7 @@ std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::
     const fe *fri_rows_dev = upload(c, d_fri_rows, fri_rows);
     for (size_t d = 0; d < P.layers.size(); d++)
         if (!P.layers[d].values.empty())
-            hash64_contiguous(c, fri_rows_dev + 4 * fri_off[d], pool_dev + 2 * (size_t)fv_base[d], P.layers[d].values.size());
+            hash64_contiguous<H>(c, fri_rows_dev + 4 * fri_off[d], pool_dev + 2 * (size_t)fv_base[d], P.layers[d].values.size());
 
     // ---- device: all Merkle plans
     std::vector<uint32_t> ops, level_start;
@@ -439,7 +434,7 @@ std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::
     const uint32_t *ops_dev = upload(c, d_ops, ops);
     const uint32_t *ls_dev = upload(c, d_ls, level_start);
     const TreeDesc *trees_dev = upload(c, d_trees, trees);
-    merkle_verify_kernel<<<(unsigned)trees.size(), 128, 0, c.stream>>>(pool_dev, ops_dev, ls_dev, trees_dev); c.launches++;
+    merkle_verify_kernel<H><<<(unsigned)trees.size(), 128, 0, c.stream>>>(pool_dev, ops_dev, ls_dev, trees_dev); c.launches++;
     DG_CUDA(cudaGetLastError());
 
     // ---- 4: constraints at z (verifier.rs:47-52, 79-97)
@@ -623,6 +618,16 @@ std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::
     }
     if (!fri_err.empty()) return "verification of low-degree proof failed: " + fri_err;
     return "";
+}
+}  // namespace
+
+// returns "" when the proof is accepted, the reference's error string otherwise; throws Error for malformed input / CUDA failures
+std::string verify_proof(Context &c, const uint8_t program_hash[32], const std::vector<fe> &inputs, const std::vector<fe> &outputs,
+                         const uint8_t *proof_bytes, size_t proof_len) {
+    ParsedProof P;
+    if (!parse_proof(proof_bytes, proof_len, P)) throw Error(DG_ERR_INVALID, "malformed proof bytes (bincode layout of StarkProof, proof.rs:10-37)");
+    if (P.hash_id != Blake3Hash::id && P.hash_id != Sha3Hash::id) return "unsupported hash function";
+    return with_proof_hash(P.hash_id, [&](auto h) { return verify_parsed<decltype(h)>(c, P, program_hash, inputs, outputs); });
 }
 
 }  // namespace dg

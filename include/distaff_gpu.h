@@ -54,7 +54,7 @@ typedef struct {                   /* ProofOptions (options.rs:16-23) */
     uint32_t extension_factor;     /* 16..256, power of two (default 32) */
     uint32_t num_queries;          /* 1..128 (default 50)                */
     uint32_t grinding_factor;      /* 0..32 (default 20)                 */
-    uint32_t hash_id;              /* 0 = blake3 (the only serialisable hash, options.rs:107) */
+    uint32_t hash_id;              /* DG_HASH_BLAKE3 (0, default) or DG_HASH_SHA3 (4): the hash of every commitment of the proof */
 } dg_options_t;
 
 typedef struct dg_proof dg_proof_t;
@@ -91,7 +91,10 @@ typedef struct {
 } dg_rng_callbacks_t;
 int dg_set_rng_callbacks(const dg_rng_callbacks_t *callbacks);
 
-/* bincode 1.3.1 encoding of StarkProof (proof.rs:10-37), what main.rs:45 serialises */
+/* bincode 1.3.1 encoding of StarkProof (proof.rs:10-37), what main.rs:45 serialises.  Its last byte is the hash id of the options
+ * (the last field of StarkProof): 0 for blake3.  A sha3 proof is written in the same layout with that byte set to 4 -- an extension of
+ * this interface: the reference's serializer refuses sha3 (options.rs:97-120), so a Rust caller deserialises such bytes with the byte
+ * set to 0 and restores the options it proved with (INTEGRATION.md section 2).  dg_verify reads the byte back the same way. */
 int dg_proof_serialized_len(const dg_proof_t *proof, size_t *len);
 int dg_proof_serialize(const dg_proof_t *proof, uint8_t *buf, size_t cap);
 /* intermediate commitments, for differential tests: which = 0 trace root, 1 constraint root, 2 PoW seed */
@@ -121,12 +124,15 @@ int dg_merkle_build(const uint8_t *leaves, uint64_t n_leaves, uint8_t *nodes);
 int dg_hash_rows(const uint8_t *columns, uint32_t width, uint64_t rows, uint8_t *digests);
 /* utils::find_pow_nonce (proof_of_work.rs:4-32) */
 int dg_find_pow_nonce(const uint8_t seed[32], uint32_t grinding_factor, uint64_t *nonce, uint8_t new_seed[32]);
-/* crypto::hash::{blake3, rescue, poseidon} (hash.rs:119-177,205-209) over n independent 64-byte messages -> n 32-byte digests
- * (benches/hash.rs), and build_merkle_nodes (merkle.rs:269-294) with any of them.  hash: 0 blake3, 1 rescue, 2 poseidon -- ids of
- * THIS interface; a proof can only carry blake3 (options.rs:97-125).  Messages must hold valid field elements for 1 and 2 (field.rs:25). */
+/* crypto::hash::{blake3, rescue, poseidon, sha3} (hash.rs:119-177,205-218) over n independent 64-byte messages -> n 32-byte digests
+ * (benches/hash.rs), and build_merkle_nodes (merkle.rs:269-294) with any of them.  hash: 0 blake3, 1 rescue, 2 poseidon, 4 sha3 (SHA3-256)
+ * -- ids of THIS interface (3 is GMiMC, which has no GPU kernel).  A proof can carry blake3 or sha3 (dg_options_t.hash_id): rescue,
+ * poseidon and GMiMC absorb at most 64 bytes and a trace row is longer, so the reference panics when it commits with them.
+ * Messages must hold valid field elements for 1 and 2 (field.rs:25). */
 #define DG_HASH_BLAKE3 0
 #define DG_HASH_RESCUE 1
 #define DG_HASH_POSEIDON 2
+#define DG_HASH_SHA3 4
 int dg_hash64(int hash, const uint8_t *messages64, uint64_t n, uint8_t *digests32);
 int dg_merkle_build_with(int hash, const uint8_t *leaves, uint64_t n_leaves, uint8_t *nodes);
 /* element-wise field ops on vectors (op: 0 add, 1 sub, 2 mul, 3 inv, 4 exp(a, b)), for differential tests of the arithmetic;
@@ -167,6 +173,8 @@ int dg_host_prng_vector(const uint8_t seed[32], uint64_t count, uint8_t *out16);
 int dg_host_query_positions(const uint8_t seed[32], uint64_t domain_size, uint32_t extension_factor, uint32_t num_queries, uint64_t *out);
 /* blake3 of a message of at most 1024 bytes (the FRI-roots seed of prover.rs:119-127) */
 int dg_host_blake3(const uint8_t *data, size_t len, uint8_t out32[32]);
+/* SHA3-256 (FIPS 202) of a message of any length: the FRI-roots seed of a sha3 proof */
+int dg_host_sha3(const uint8_t *data, size_t len, uint8_t out32[32]);
 /* MerkleTree::prove_batch planning (merkle.rs:64-124): writes, per normalised slot, the count and then (is_leaf, index) pairs;
  * out layout: [n_slots][depth] then for each slot [count] (is_leaf, index)*count, all uint64 */
 int dg_host_plan_batch(const uint64_t *indexes, uint32_t n_indexes, uint64_t n_leaves, uint64_t *out, size_t cap, size_t *written);

@@ -1,11 +1,13 @@
 #!/usr/bin/env python3
 """Multi-GPU parity check (run under torchrun): one proof sharded over WORLD_SIZE GPUs must be byte-identical to the CPU oracle's.
-    torchrun --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/multi_gpu_check.py"""
+    torchrun --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/multi_gpu_check.py [--hash sha3]
+--hash picks the commitment hash of every proof (default blake3)."""
 import os
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+HASH = sys.argv[sys.argv.index("--hash") + 1] if "--hash" in sys.argv else "blake3"
 rank, local_rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 os.environ["DG_DEVICE"] = str(local_rank)
 import torch                       # noqa: E402
@@ -13,7 +15,7 @@ import torch.distributed as dist   # noqa: E402
 import distaff_b200 as dg          # noqa: E402
 from distaff_b200 import backend, hostvm   # noqa: E402
 from oracle import pyoracle as po  # noqa: E402
-from tests import programs         # noqa: E402
+from tests import programs, sha3_oracle as so   # noqa: E402
 
 torch.cuda.set_device(local_rank)
 if world > 1:
@@ -25,9 +27,13 @@ for name, tr in cases:
     for opts in ((32, 50, 20),) + (((64, 20, 8), (128, 10, 4)) if name in ("collatz3", "fib13") else ()):
         if opts[0] // world < 4:
             continue
-        p = dg.prove(tr, dg.ProofOptions(*opts))
-        ref = po.prove(tr.registers, tr.ctx_depth, tr.loop_depth, tr.public_inputs, tr.outputs, ext=opts[0], num_queries=opts[1], grinding=opts[2])
-        same = p.bytes == ref.proof
+        p = dg.prove(tr, dg.ProofOptions(*opts, hash_fn=HASH))
+        if HASH == "sha3":
+            ref = so.prove(tr.registers, tr.ctx_depth, tr.loop_depth, tr.public_inputs, tr.outputs, ext=opts[0], num_queries=opts[1], grinding=opts[2])
+        else:
+            ref = po.prove(tr.registers, tr.ctx_depth, tr.loop_depth, tr.public_inputs, tr.outputs, ext=opts[0], num_queries=opts[1],
+                           grinding=opts[2]).proof
+        same = p.bytes == ref
         ok &= same
         if rank == 0:
             print(f"[world {world}] {name} {opts}: identical={same} len={len(p.bytes)} ms={p.stats['total_ms']:.2f}", flush=True)
@@ -37,7 +43,7 @@ regs = tr.registers.copy()
 regs[tr.width - 1, 100, 0] += 1
 bad = hostvm.ExecutionTrace(regs, tr.ctx_depth, tr.loop_depth, tr.stack_depth, tr.program_hash, tr.public_inputs, tr.outputs)
 try:
-    dg.prove(bad)
+    dg.prove(bad, dg.ProofOptions(hash_fn=HASH))
     ok = False
     print(rank, "invalid trace was proven!?")
 except backend.DgError as e:
